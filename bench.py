@@ -121,6 +121,27 @@ class ClockSampler:
                 "source": "nvml" if self._nvml else "nvidia-smi"}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(d, arrays):
+    """Write each array as ``d/<name>.npy`` (floats as float32 / float64, integer ids as float64, exact below 2**53) so that
+    two builds can be compared output for output.  An array larger than its share of DUMP_BYTES is replaced by a fixed,
+    seeded sample of its elements (same indices for the same shape)."""
+    import numpy as np
+    import torch
+    os.makedirs(d, exist_ok=True)
+    share = DUMP_BYTES // max(len(arrays), 1)
+    for name, t in arrays.items():
+        t = torch.as_tensor(t).detach()
+        a = t.double() if (not t.is_floating_point() or t.dtype == torch.float64) else t.float()
+        a = a.cpu().numpy()
+        if a.nbytes > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 def count_own_launches(trainer):
     """Kernel launches of one step, split into ours (namespace glb::) and library kernels."""
     import torch
@@ -215,7 +236,7 @@ def build_trainer(args, rt, shape, feature_dtype, cache_rows_arg):
     return tr, nodes, csr, cache_rows, build_s, g
 
 
-def time_trainer(args, rt, tr, nodes, steps, clocks=None):
+def time_trainer(args, rt, tr, nodes, steps, clocks=None, dump_dir=None):
     """(device-timed ms, e2e ms, last loss).  Device region: K graph replays, every one samples a FRESH seed batch
     (already resident on the device).  End-to-end region: the public step - host seeds (GSL traversal when built
     from a query) -> pinned staging -> H2D inside the step graph, loss -> pinned host every step."""
@@ -270,6 +291,13 @@ def time_trainer(args, rt, tr, nodes, steps, clocks=None):
     final_loss = float(last)
     if hasattr(tr, "ar"):
         tr.ar.check()
+    if dump_dir and rt.rank == 0:
+        # the last step's loss as the caller received it, the logits of that step's seed batch, the updated weights
+        outs = {"loss": last}
+        if hasattr(tr, "H"):
+            outs["logits"] = tr.H[-1]
+        outs.update(("param." + n, p) for n, p in tr.model.named_parameters())
+        dump_outputs(dump_dir, outs)
     t = torch.tensor([ms_dev, ms_e2e], device=rt.device, dtype=torch.float64)
     if W > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -295,7 +323,7 @@ def run_ours(args):
     # ---- headline: hash-partitioned graph, NO replica cache: every remote row crosses NVLink inside the fused kernel
     tr, nodes, csr, cache_rows, build_s, g = build_trainer(args, rt, shape, args.feature_dtype, args.feature_cache_rows)
     clocks = ClockSampler(rt.local_rank) if rt.rank == 0 else None
-    ms_dev, ms_e2e, final_loss = time_trainer(args, rt, tr, nodes, args.steps, clocks)
+    ms_dev, ms_e2e, final_loss = time_trainer(args, rt, tr, nodes, args.steps, clocks, args.dump_outputs)
     clk = clocks.stop() if clocks else None
     own, lib, names = count_own_launches(tr)
     # payload bytes of a feature row (the 128-byte aligned stride adds padding that is never read)
@@ -425,10 +453,12 @@ def run_walks(args, rt):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record()
     for i in range(args.steps):
-        one(warm + i)
+        walks, neg = one(warm + i)
     ev1.record()
     torch.cuda.synchronize(); rt.barrier()
     ms_dev = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rt.rank == 0:
+        dump_outputs(args.dump_outputs, {"walks": walks, "neg": neg})
     # e2e through the public API
     q = g.V("n").batch(B).shuffle(traverse=True).alias("src").random_walk("e", L).alias("walk") \
          .outNeg("e").sample(NEGS).by("random").alias("neg").values()
@@ -590,6 +620,10 @@ def run_bipartite_gat(args, rt):
     ev1.record()
     torch.cuda.synchronize(); rt.barrier()
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rt.rank == 0:
+        outs = {"loss": last}
+        outs.update(("param." + n, p) for n, p in model.named_parameters())
+        dump_outputs(args.dump_outputs, outs)
     clk = clocks.stop() if clocks else None
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if W > 1:
@@ -651,6 +685,11 @@ def main():
                     help="gsl = in-memory sources -> gl.Graph -> GSL query -> compiled plan -> engine; raw = shards handed to the trainer")
     ap.add_argument("--no-secondary", action="store_true", help="skip the labelled secondary run (replica cache / other row dtype)")
     ap.add_argument("--small", action="store_true", help="small graph for quick functional runs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step returned (loss, logits, updated weights; walks and "
+                         "negatives for deepwalk) as DIR/<name>.npy; the inputs are seeded, so two builds compare file for file. "
+                         "Float atomics (loss, bias gradients) round in a run-dependent order and Adam amplifies that over the "
+                         "steps: compare trained outputs with a tolerance, or with few --steps")
     args = ap.parse_args()
     args.cfg = CONFIGS[args.config]
     world = int(os.environ.get("WORLD_SIZE", "1"))
